@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (+ what the last timed step returned, DIR/<name>.npy)
 
 Workload (BASELINE.json configs[1], SURVEY.md 8d "Config 2"): 4 096 SMPL envs per GPU, env=speed, flat ground,
 state_init=Default, self_obs_v=1 (obs 292), control_mode=uhc_pd (the reference's yaml default: stable PD), actions
@@ -60,6 +61,7 @@ def make_cfg(wl=None):
     return mk(env=w["env"], robot=w["robot"], overrides=w["overrides"])
 
 
+DUMP_BYTES = 64 * 10 ** 6           # --dump-outputs: at most this much in all
 PEAK_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12     # 148 SMs x 128 FP32 lanes x 2 (FMA) x clocks.max.sm: 74.5 TFLOP/s nominal
 
 
@@ -119,6 +121,20 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": float(max(mx)) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(path, outs):
+    """Write each array of `outs` ([envs, ...], float32) as path/<name>.npy.  Above DUMP_BYTES in all, a fixed seeded sample of the
+    envs is written instead, with their indices in env_ids.npy."""
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(outs.values())))
+    row = sum(a[0].nbytes for a in outs.values()) + 8
+    if n * row > DUMP_BYTES:
+        ids = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row, replace=False))
+        outs = {k: a[ids] for k, a in outs.items()}
+        outs["env_ids"] = ids.astype(np.float64)
+    for k, a in outs.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 def measured_peak_hbm():
@@ -274,12 +290,13 @@ def measure(wl, args, torch, dist, world, rank, local, K, W, headline):
     def one_step(a):
         if motion:   # reference-pose feed of the step (motion_lib_base.py:313-354), then the step, then MoCap reset of finished envs
             st = lib.get_motion_state_intervaled(ids, t_env)
-            env.step(a)
+            out = env.step(a)
             env.reset(env.reset_buf, init_mode=2, qpos0=st["qpos"], qvel0=st["qvel"])
             t_env.add_(dt)
             t_env.masked_fill_(t_env > 9.0, 0.0)
         else:
-            env.step(a); env.reset_done()
+            out = env.step(a); env.reset_done()
+        return out
 
     if motion:
         st0 = lib.get_motion_state_intervaled(ids, t_env)
@@ -299,10 +316,14 @@ def measure(wl, args, torch, dist, world, rank, local, K, W, headline):
     barrier()
     ev0.record()
     for i in range(K):
-        one_step(acts[i]); flush.zero_()
+        last = one_step(acts[i]); flush.zero_()
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    # what the caller holds after the last timed step (obs after the in-stream reset of the envs that finished), before the
+    # kernel timing below steps the env again
+    outputs = {k: t.float().cpu().numpy() for k, t in zip(("obs", "reward", "terminated", "truncated"), last)} \
+        if headline and args.dump_outputs else None
     launches = env.gpu_launches - launches0
     # ---------------- the L2 flush alone (it sits inside the timed region above: `value` is conservative by this much)
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -356,7 +377,8 @@ def measure(wl, args, torch, dist, world, rank, local, K, W, headline):
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms, e2e_ms, k_ms, flush_ms = [float(x) for x in t.tolist()]
-    out = dict(N=N, K=K, ms=ms, e2e_ms=e2e_ms, Ke=Ke, k_ms=k_ms, flush_ms=flush_ms, launches=launches, clocks=clocks, env=env, cfg=cfg)
+    out = dict(N=N, K=K, ms=ms, e2e_ms=e2e_ms, Ke=Ke, k_ms=k_ms, flush_ms=flush_ms, launches=launches, clocks=clocks, env=env, cfg=cfg,
+               outputs=outputs)
     return out
 
 
@@ -416,7 +438,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-extra", action="store_true", help="skip the short cfg4 / cfg5 runs appended to the headline line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (obs, reward, terminated, truncated) "
+                                                          "as DIR/<name>.npy in float32; same arguments, same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     global _WL, WORKLOAD, B_ALG_BYTES
     _WL = args.workload
     WORKLOAD, B_ALG_BYTES = WORKLOADS[_WL]["desc"], WORKLOADS[_WL]["balg"]
@@ -450,6 +478,8 @@ def main():
             del x
         extra["ppo"] = measure_ppo(torch, dist, world, rank, local)
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         ms, e2e_ms, k_ms, Ke = r["ms"], r["e2e_ms"], r["k_ms"], r["Ke"]
         nu = env.num_actions
         total_envs = N * world

@@ -29,3 +29,20 @@ def test_reference_arm_prints_one_json_line():
 
 def test_reference_arm_other_ranks_are_silent():
     assert _run({"RANK": "1", "WORLD_SIZE": "2"}) == []
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_envs_above_the_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(1)
+    outs = {"obs": rng.normal(size=(50, 7)).astype(np.float32), "reward": rng.random(50).astype(np.float32)}
+    bench.dump_outputs(str(tmp_path / "all"), outs)
+    assert sorted(os.listdir(tmp_path / "all")) == ["obs.npy", "reward.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "obs.npy"), outs["obs"])
+    monkeypatch.setattr(bench, "DUMP_BYTES", 20 * (8 * 4 + 8))          # room for 20 of the 50 envs
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    ids = np.load(tmp_path / "a" / "env_ids.npy")
+    assert ids.dtype == np.float64 and len(ids) == 20 and np.array_equal(ids, np.load(tmp_path / "b" / "env_ids.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "obs.npy"), outs["obs"][ids.astype(int)])
+    assert sum(os.path.getsize(tmp_path / "a" / f) - 128 for f in os.listdir(tmp_path / "a")) <= bench.DUMP_BYTES

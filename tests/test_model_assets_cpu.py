@@ -1,27 +1,27 @@
 """The shipped constant tables (smplsim_b200/assets/*.model.json) are *derived* from the reference's MJCF files by the in-repo parser
-(tools/extract_model.py).  Where the reference tree is present (build container) a fresh parse must reproduce them exactly; the MJCF
-parser itself is exercised on a small hand-written model everywhere."""
+(tools/extract_model.py).  They must equal what a fresh parse of those XMLs gave (tests/golden/model_tables.npz, written by
+tests/golden/make_golden_model_tables.py); the MJCF parser itself is exercised on a small hand-written model."""
 import os
 
 import numpy as np
 import pytest
 
+from conftest import GOLDEN
 from smplsim_b200.mjcf import parse_mjcf
 from smplsim_b200.model import build_model, load_model
 
-REF = os.environ.get("SMPLSIM_REFERENCE", "/root/reference")
-XMLS = {"smpl": os.path.join(REF, "smpl_sim/data/assets/mjcf/smpl_humanoid.xml"), "smplx": os.path.join(REF, "smpl_humanoid.xml")}
+FIELDS = ("body_parent", "body_pos", "body_quat", "body_mass", "body_ipos", "body_inertia", "dof_armature", "dof_range", "dof_invweight0",
+          "geom_type", "geom_body", "geom_pos", "geom_mat", "geom_size", "act_kp", "act_kd", "act_torque_lim", "act_scale", "act_offset")
 
 
 @pytest.mark.parametrize("name", ["smpl", "smplx"])
 def test_shipped_tables_equal_fresh_parse_of_reference_xml(name):
-    if not os.path.exists(XMLS[name]):
-        pytest.skip("reference tree not present (GPU box): the shipped tables are used as they are")
-    a, b = load_model(name), load_model(XMLS[name])
-    assert a.body_names == b.body_names and a.joint_names == b.joint_names and a.geom_names == b.geom_names
-    for f in ("body_parent", "body_pos", "body_quat", "body_mass", "body_ipos", "body_inertia", "dof_armature", "dof_range", "dof_invweight0",
-              "geom_type", "geom_body", "geom_pos", "geom_mat", "geom_size", "act_kp", "act_kd", "act_torque_lim", "act_scale", "act_offset"):
-        x, y = np.asarray(getattr(a, f)), np.asarray(getattr(b, f))
+    g = np.load(os.path.join(GOLDEN, "model_tables.npz"))
+    a = load_model(name)
+    for f in ("body_names", "joint_names", "geom_names"):
+        assert list(getattr(a, f)) == g[f"{name}.{f}"].tolist(), f
+    for f in FIELDS:
+        x, y = np.asarray(getattr(a, f)), g[f"{name}.{f}"]
         assert x.shape == y.shape and np.allclose(x, y, rtol=0, atol=1e-12), f
 
 
